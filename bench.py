@@ -15,6 +15,10 @@ Prints ONE JSON line (rank 0).  `value` has the PCM already resident in HBM;
 `e2e` goes through Analyzer.fingerprint_packed with pinned HOST buffers, the
 host->device copy of the PCM and the device->host read of the hashes inside the
 timed region.
+
+--dump-outputs DIR writes what the timed steps computed in their last step as .npy
+files (see dump_outputs), so that two builds can be compared output for output: the
+synthetic input is a fixed function of the arguments.
 """
 from __future__ import annotations
 
@@ -83,10 +87,10 @@ _TRACKS = None      # set before the CPU pool is forked: workers inherit the PCM
 
 
 def reference_dir():
-    """A checkout of the reference (dpwe/audfprint) if one is reachable: $AFP_REFERENCE,
-    baseline/_ref, /root/reference.  It is pure Python and is NOT part of this repo, so on the
-    GPU box there is normally none and the CPU arm is the oracle port (`kind: "port"`)."""
-    for d in (os.environ.get("AFP_REFERENCE"), os.path.join(ROOT, "baseline", "_ref"), "/root/reference"):
+    """A checkout of the reference (dpwe/audfprint) if one is reachable: $AFP_REFERENCE or
+    baseline/_ref.  It is pure Python and is NOT part of this repo; without one the CPU arm is
+    the oracle port (`kind: "port"`)."""
+    for d in (os.environ.get("AFP_REFERENCE"), os.path.join(ROOT, "baseline", "_ref")):
         if d and os.path.isfile(os.path.join(d, "audfprint_analyze.py")):
             return d
     return None
@@ -314,7 +318,7 @@ def bench_match(a, an, ctx, tracks, rows, roff, queries, cores, want_cpu, stream
     res = m.match_batch(ht, (qrows, qoff))
     warm_up(lambda: m.match_batch(ht, (qrows, qoff)))
     # --- match only, host hashes in / rows out (includes H2D of the query hashes, D2H of rows)
-    steps = 5
+    steps = a.steps
     torch.cuda.synchronize()
     t0 = time.perf_counter()
     for _ in range(steps):
@@ -406,7 +410,7 @@ def bench_match(a, an, ctx, tracks, rows, roff, queries, cores, want_cpu, stream
                                "sample": "%d of the %d queries, oracle port (Python loop over query hashes as "
                                          "the reference) on a %d-process pool, %.1f s wall" % (ns, nq, min(cores, ns), dt)}
         out["parity"] = {"queries_checked": ns, "queries_mismatched": bad}
-    return out
+    return out, res
 
 
 def bench_match_sharded(a, an, rows, roff, qpool, rank, world):
@@ -464,10 +468,10 @@ def bench_match_sharded(a, an, rows, roff, qpool, rank, world):
     dist.barrier()
     torch.cuda.synchronize()
     t0 = time.perf_counter()
-    for _ in range(3):       # query hashes resident, rows left on the device - like the N=1 `value`
+    for _ in range(a.steps):       # query hashes resident, rows left on the device - like the N=1 `value`
         ctx.check(ctx.lib.afp_match_batch(ctx.h, dq.data_ptr(), 0, len(mine), offp, C.byref(pp), C.byref(tot)))
     torch.cuda.synchronize()
-    dtr = torch.tensor([(time.perf_counter() - t0) / 3], dtype=torch.float64, device="cuda")
+    dtr = torch.tensor([(time.perf_counter() - t0) / a.steps], dtype=torch.float64, device="cuda")
     dist.all_reduce(dtr, op=dist.ReduceOp.MAX)
     rep_bad = 0
     if rank == 0:
@@ -479,7 +483,7 @@ def bench_match_sharded(a, an, rows, roff, qpool, rank, world):
     dbatches = [(torch.from_numpy(qb[0]).cuda(), qb[1]) for qb in batches]   # query hashes resident, like the N=1 `value`
     for k in range(24):         # collective calls: the same count on every rank; ~0.4 s of GPU work
         afd.match_sharded_batch(m, ht, dbatches[k % len(dbatches)], row_cap=16, fetch=False)
-    steps = 3
+    steps = a.steps
     dist.barrier()
     torch.cuda.synchronize()
     t0 = time.perf_counter()
@@ -676,6 +680,46 @@ def bench_ingest(a, rank, local_rank, world, cores, pool):
     return 0
 
 
+# ---------------------------------------------------------------- --dump-outputs
+def fetch_last_hashes(ctx, nfiles):
+    """(rows, row_offsets) of the last fingerprint batch, read back from the context's workspace
+    (what Analyzer.fingerprint_packed returns with fetch=True)."""
+    import ctypes as C
+    roff = np.empty(nfiles + 1, np.int64)
+    ctx.check(ctx.lib.afp_fetch_hashes(ctx.h, None, 1, roff.ctypes.data_as(C.POINTER(C.c_int64))))
+    rows = np.empty((int(roff[-1]), 2), np.int32)
+    ctx.check(ctx.lib.afp_fetch_hashes(ctx.h, rows.ctypes.data, 1, None))
+    return rows, roff
+
+
+def dump_outputs(d, groups, limit=64 << 20, seed=0):
+    """Write ragged int results as float64 .npy files under `d` (every value is exact in float64).
+    `groups` maps a name to (rows, offsets), the rows of item i (a file, a query) being
+    rows[offsets[i]:offsets[i + 1]].  A group gives d/<name>.npy (the rows of the items written,
+    one item after the other), d/<name>_offsets.npy and d/<name>_items.npy (the item indices).
+    All items are written when the files fit in `limit` bytes; otherwise every group is cut to
+    a seeded random sample of whole items, the same for the same arguments, that fits."""
+    os.makedirs(d, exist_ok=True)
+    rng = np.random.default_rng(seed)
+    sizes = {name: 8 * (rows.size + 2 * len(off)) for name, (rows, off) in groups.items()}
+    total = sum(sizes.values())
+    for name, (rows, off) in groups.items():
+        off = np.asarray(off, np.int64)
+        lens = np.diff(off)
+        items = np.arange(len(lens))
+        if total > limit:
+            order = rng.permutation(len(lens))
+            cost = np.cumsum(8 * (lens[order] * rows.shape[1] + 2))
+            budget = (limit - 3 * 128 * len(groups)) * sizes[name] // total - 8     # 128-byte .npy headers
+            items = np.sort(order[cost <= budget])
+        n = lens[items]
+        start = np.cumsum(n) - n
+        idx = np.repeat(off[items], n) + np.arange(int(n.sum())) - np.repeat(start, n)
+        np.save(os.path.join(d, name + ".npy"), rows[idx].astype(np.float64))
+        np.save(os.path.join(d, name + "_offsets.npy"), np.concatenate([[0], np.cumsum(n)]).astype(np.float64))
+        np.save(os.path.join(d, name + "_items.npy"), items.astype(np.float64))
+
+
 def measured_peaks():
     try:
         with open(os.path.join(ROOT, "MEASURED_PEAKS.json")) as f:
@@ -687,11 +731,11 @@ def measured_peaks():
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 10; 12 with --config 3)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--files", type=int, default=1024, help="files per GPU per step")
-    ap.add_argument("--seconds", type=float, default=30.0)
+    ap.add_argument("--seconds", type=float, default=None, help="seconds per file (default 30; 180 with --config 3)")
     ap.add_argument("--cpu-sample", type=int, default=512, help="files in the CPU-baseline sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true",
@@ -707,12 +751,17 @@ def main():
                          "queries on 1 GPU, 3 ingest 180 s tracks incl. store, 4 sharded-table match of 100k queries")
     ap.add_argument("--match-cpu-sample", type=int, default=1024,
                     help="queries in the CPU baseline / parity sample of the match leg (~3 s on 16 cores)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the hashes (and match rows) of the last timed step as .npy files under DIR")
     a = ap.parse_args()
     if a.match_queries is None:
         a.match_queries = 100000 if a.config == 4 else 10000
-    if a.config == 3:
-        a.seconds = 180.0 if a.seconds == 30.0 else a.seconds
-        a.steps = 12 if a.steps == 10 else a.steps
+    if a.steps is None:
+        a.steps = 12 if a.config == 3 else 10
+    if a.seconds is None:
+        a.seconds = 180.0 if a.config == 3 else 30.0
+    if a.dump_outputs and (a.impl == "reference" or a.config in (3, 4)):
+        ap.error("--dump-outputs writes the outputs of --config 1 and 2 of this implementation")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -838,6 +887,7 @@ def main():
     clocks = sampler.stop()
     ctx.set_profiling(False)
     stages /= a.steps
+    last_step = fetch_last_hashes(ctx, a.files) if a.dump_outputs and rank == 0 else None
 
     # ---- end to end: pinned host PCM in, hashes + offsets out, every step --------------------
     rows, roff = an.fingerprint_packed(dev_pcm, offs, sample_lengths=lens)
@@ -948,9 +998,9 @@ def main():
             config0["identical_to_cpu_path"] = bool(np.array_equal(h0, orc.fingerprint(pcm_to_float(clip))))
             config0["cpu_single_core"] = config0_single_core()
 
-    match = None
+    match, match_rows = None, None
     if do_match and world == 1:
-        match = bench_match(a, an, ctx, tracks, rows, roff, queries, cores, want_cpu, stream)
+        match, match_rows = bench_match(a, an, ctx, tracks, rows, roff, queries, cores, want_cpu, stream)
     elif do_match:
         match = bench_match_sharded(a, an, rows, roff, qpool, rank, world)
 
@@ -991,7 +1041,7 @@ def main():
             # BASELINE configs[2] / configs[4]: the match leg is the headline line, the fingerprint
             # numbers of the same run ride along
             line = dict(match)
-            line.update({"n_gpus": world, "steps": 3 if world > 1 else 5, "warmup": 2, "higher_is_better": True,
+            line.update({"n_gpus": world, "steps": a.steps, "warmup": 2, "higher_is_better": True,
                          "scaling": "strong" if world > 1 else "weak", "vs_baseline": None, "dtype": "u32",
                          "data": "synthetic", "clocks": clocks, "gpu_launches": 2,
                          "config": {"workload": ("match %d x 10 s noisy synthetic queries (4 shifts) against a "
@@ -1004,6 +1054,12 @@ def main():
             print(json.dumps(line))
         else:
             print(json.dumps(out))
+    if last_step is not None:
+        groups = {"hashes": last_step}                  # (time, hash) rows of every file
+        if match_rows is not None:                      # (id, count, offset, ...) rows of every query
+            groups["match_rows"] = (np.concatenate(match_rows).reshape(-1, 7),
+                                    np.concatenate([[0], np.cumsum([len(r) for r in match_rows])]))
+        dump_outputs(a.dump_outputs, groups)
     if world > 1:
         dist.destroy_process_group()
     if cpool:

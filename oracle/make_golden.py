@@ -151,7 +151,11 @@ def main():
                 print(db, cfg, key, "nq", len(q), "hits", len(hits), "nrows", len(rows),
                       "top", rows[:1].tolist(), "truth", m[key + "/truth"][0],
                       m[key + "/truth"][1] // 256, "ties", tie_w, tie_c)
-    np.savez_compressed(os.path.join(OUT, "match.npz"), **m)
+    # the hits go to a file of their own, column-major (it compresses better), so that each
+    # file stays under 1 MB; tests.conftest.load_golden joins the two
+    np.savez_compressed(os.path.join(OUT, "match_hits.npz"),
+                        **{k: np.asfortranarray(v) for k, v in m.items() if k.endswith("/hits")})
+    np.savez_compressed(os.path.join(OUT, "match.npz"), **{k: v for k, v in m.items() if not k.endswith("/hits")})
 
     # a small database saved by the reference's own HashTable.save (gzip pickle of the object,
     # hash_table.py:178-197): the mirror class must load it (tests/test_abi_cpu.py)

@@ -13,9 +13,9 @@ the live reference runs on that PCM with its reader replaced by the decoder.
 Run in the build container only (the GPU box has no /root/reference):
     python oracle/make_golden_bundled.py
 Stored in tests/golden/bundled.npz: reference OUTPUTS (hashes, table rows,
-match rows, report lines) and the decoded int16 PCM of the query and of
-PCM_TRACKS (the input the GPU parity tests need; the GPU box has neither the
-MP3s nor /root/reference).  No reference source is copied.
+match rows, report lines); in tests/golden/bundled_pcm.npz: the decoded int16
+PCM of the query and of PCM_TRACKS (the input the GPU parity tests need, where
+neither the MP3s nor the reference are at hand).  No reference source is copied.
 """
 from __future__ import annotations
 
@@ -170,8 +170,11 @@ def main():
         for nm, src in (("query", short(query)), ("track4", short(files[4]))):
             pk = pan.wavfile2peaks(src)
             g["%s/%s/peaks" % (tag, nm)] = np.asarray(pk, np.int32).reshape(-1, 2)
-    np.savez_compressed(OUT, **g)
-    print("wrote", OUT, os.path.getsize(OUT), "bytes")
+    pcm_out = OUT.replace(".npz", "_pcm.npz")          # each file stays under 1 MB
+    np.savez_compressed(pcm_out, **{k: v for k, v in g.items() if k.endswith("/pcm")})
+    np.savez_compressed(OUT, **{k: v for k, v in g.items() if not k.endswith("/pcm")})
+    for fn in (OUT, pcm_out):
+        print("wrote", fn, os.path.getsize(fn), "bytes")
 
 
 if __name__ == "__main__":

@@ -20,9 +20,19 @@ def golden_fp():
     return np.load(os.path.join(GOLDEN, "fingerprint.npz"))
 
 
+def load_golden(*names):
+    """The arrays of tests/golden/<name>.npz for every name, in one mapping (a set of vectors is
+    split over several files to keep each of them under 1 MB)."""
+    out = {}
+    for name in names:
+        with np.load(os.path.join(GOLDEN, name + ".npz")) as g:
+            out.update((k, np.asarray(g[k], order="C")) for k in g.files)
+    return out
+
+
 @pytest.fixture(scope="session")
 def golden_match():
-    return np.load(os.path.join(GOLDEN, "match.npz"))
+    return load_golden("match", "match_hits")
 
 
 @pytest.fixture(scope="session")

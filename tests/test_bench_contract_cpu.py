@@ -20,8 +20,9 @@ def test_reference_arm_prints_the_contract_line():
     assert d["impl"] == "reference" and d["metric"] == "audio_seconds_fingerprinted_per_sec"
     assert d["unit"] == "audio-s/s" and d["higher_is_better"] is True and d["n_gpus"] == 1
     assert d["steps"] == 1 and d["warmup"] == 1 and d["value"] > 0 and d["ms_per_step"] > 0
-    # the unmodified reference where a checkout is reachable (build container), the oracle port otherwise
-    want_kind = "reference" if os.path.isfile("/root/reference/audfprint_analyze.py") else "port"
+    # the unmodified reference where a checkout is reachable, the oracle port otherwise
+    refs = (os.environ.get("AFP_REFERENCE"), os.path.join(ROOT, "baseline", "_ref"))
+    want_kind = "reference" if any(d and os.path.isfile(os.path.join(d, "audfprint_analyze.py")) for d in refs) else "port"
     assert d["cpu_baseline"]["kind"] == want_kind and d["cpu_baseline"]["cores"] >= 1
     assert d["cpu_baseline"]["host_cores"]["used"] == d["cpu_baseline"]["cores"]
     assert d["config0"]["cores"] == 1 and d["config0"]["median_s"] > 0 and d["config0"]["runs"] >= 5

@@ -1,13 +1,12 @@
 """GPU: the CUDA path on the reference's OWN bundled test material (the Nine_Lives excerpts
-and query.mp3 of /root/reference/tests/data - what `make test` of the reference runs,
+and query.mp3 of the reference's tests/data - what `make test` of the reference runs,
 Makefile:12-29), against what the LIVE reference produced on the same decoded PCM
-(tests/golden/bundled.npz, oracle/make_golden_bundled.py).  BASELINE.json north_star:
-"match results bit-identical to the reference on the bundled tests/data queries".
+(tests/golden/bundled.npz and bundled_pcm.npz, oracle/make_golden_bundled.py).
+BASELINE.json north_star: "match results bit-identical to the reference on the bundled tests/data queries".
 
 Real, heavily clipped music instead of the synthetic tracks of the other tests; hashes, peaks,
 table arrays, match rows and report lines are compared bit for bit.  (The file sorts last so
 that the synthetic-input suite reports first.)"""
-import os
 import random
 
 import numpy as np
@@ -15,7 +14,7 @@ import pytest
 
 from audfprint_b200 import Analyzer, HashTable, Matcher
 from oracle import afp_oracle as orc
-from tests.conftest import GOLDEN, expand_table
+from tests.conftest import expand_table, load_golden
 
 pytestmark = pytest.mark.gpu
 PCM_TRACKS = (0, 4, 8, 12)
@@ -32,7 +31,7 @@ MATCH_CONFIGS = {           # oracle/make_golden_bundled.py
 
 @pytest.fixture(scope="module")
 def gb():
-    return np.load(os.path.join(GOLDEN, "bundled.npz"))
+    return load_golden("bundled", "bundled_pcm")
 
 
 @pytest.fixture(scope="module")

@@ -10,10 +10,11 @@ import numpy as np
 import pytest
 
 from audfprint_b200 import Analyzer, HashTable, Matcher
+from oracle import build_ref
 from tests import cases
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+REF = build_ref.reference_dir() or ""          # the reference's code, if it is at hand
 
 # What the live reference's Matcher.file_match_to_msgs returns (audfprint_match.py:381-420) when
 # match_file yields these rows; generated in the build container by patching match_file on the

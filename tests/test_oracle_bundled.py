@@ -1,14 +1,16 @@
 """CPU: the oracle against what the LIVE reference produced on its own bundled test
-material (/root/reference/tests/data: Nine_Lives/*.mp3 and query.mp3, the files of the
-reference's `make test`), stored in tests/golden/bundled.npz by
+material (the reference's tests/data: Nine_Lives/*.mp3 and query.mp3, the files of the
+reference's `make test`), stored in tests/golden/bundled.npz and bundled_pcm.npz by
 oracle/make_golden_bundled.py.  The MP3s were decoded with FFmpeg's libraries at the
 parameters of the reference's `ffmpeg -f s16le -ac 1 -ar 11025` pipe (oracle/ffdecode.py).
 
 The first group runs anywhere (committed PCM of the query and of four tracks, reference
-outputs for all thirteen).  The second group needs the reference checkout and the vendored
-FFmpeg libraries (build container only): it re-decodes the MP3s, checks the nine tracks whose
-PCM is not committed, and runs the UNMODIFIED reference command line (`new`, `add`, `match`:
-Makefile:19-29) on the decoded audio to confirm the stored report lines."""
+outputs for all thirteen).  The second group needs the reference's code and MP3s
+(oracle/_ref/, made by build() from a reference checkout, or the checkout named by
+$AFP_REFERENCE; it skips without them) and the vendored FFmpeg libraries: it re-decodes the
+MP3s, checks the nine tracks whose PCM is not committed, and runs the UNMODIFIED reference
+command line (`new`, `add`, `match`: Makefile:19-29) on the decoded audio to confirm the
+stored report lines."""
 import os
 import random
 import subprocess
@@ -18,10 +20,11 @@ import numpy as np
 import pytest
 
 from oracle import afp_oracle as orc
-from tests.conftest import GOLDEN, expand_table
+from oracle import build_ref
+from tests.conftest import expand_table, load_golden
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.environ.get("AFP_REFERENCE", "/root/reference")
+REF = build_ref.reference_dir() or ""
 PCM_TRACKS = (0, 4, 8, 12)
 DENSITIES = (100.0, 20.0)
 # Matcher settings of oracle/make_golden_bundled.py on top of the command line's defaults
@@ -38,7 +41,7 @@ CONFIGS = {
 
 @pytest.fixture(scope="module")
 def gb():
-    return np.load(os.path.join(GOLDEN, "bundled.npz"))
+    return load_golden("bundled", "bundled_pcm")
 
 
 def to_float(pcm):
@@ -138,7 +141,7 @@ def test_mirror_report_lines_from_the_reference_rows(gb):
         cases_ += [("excerpt%d" % k, "excerpt%d" % k, cfg) for k in PCM_TRACKS for cfg in ("top5", "exact_range_time", "tight")]
         for qkey, qname, cfg in cases_:
             key = "%s/%s/%s" % (tag, qkey, cfg)
-            if key + "/ties" in gb.files and any(gb[key + "/ties"]):
+            if key + "/ties" in gb and any(gb[key + "/ties"]):
                 continue
             mt = Matcher()
             mt.window, mt.threshcount, mt.max_returns, mt.search_depth = 2, 5, 1, 100
@@ -149,14 +152,14 @@ def test_mirror_report_lines_from_the_reference_rows(gb):
             an.wavfile2hashes = lambda fn, h=gb["%s/%s/hashes" % (tag, qkey)]: h
             mt.match_hashes = lambda ht, q, r=gb[key + "/rows"].astype(np.int32): r
             assert mt.file_match_to_msgs(an, Table, qname) == [str(x) for x in gb[key + "/msgs"]], key
-            if key + "/msgs_terse" in gb.files:
+            if key + "/msgs_terse" in gb:
                 mt.verbose = False
                 assert mt.file_match_to_msgs(an, Table, qname) == [str(x) for x in gb[key + "/msgs_terse"]], key
             checked += 1
     assert checked > 40
 
 
-# ---- build container only: the MP3s themselves and the live reference ------------------------
+# ---- with the reference's code and MP3s only: the MP3s themselves and the live reference ------
 def _have_decoder():
     try:
         from oracle import ffdecode
@@ -166,7 +169,7 @@ def _have_decoder():
         return False
 
 
-live = pytest.mark.skipif(not (os.path.isfile(os.path.join(REF, "tests", "data", "query.mp3")) and _have_decoder()),
+live = pytest.mark.skipif(not (REF and os.path.isfile(os.path.join(REF, "tests", "data", "query.mp3")) and _have_decoder()),
                           reason="needs the reference checkout and the vendored FFmpeg libraries")
 
 

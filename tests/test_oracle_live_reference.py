@@ -1,62 +1,35 @@
-"""CPU, build container only: the oracle against the LIVE reference on seeds that are not in
-tests/golden (skipped where /root/reference does not exist, i.e. on the GPU box).  The reference
-is imported in a subprocess so that its module names (hash_table, ...) never enter this process."""
-import json
+"""CPU: the oracle against what the reference produced on seeds and parameter settings that
+the other golden files do not cover (tests/golden/live_reference.npz, written by
+oracle/make_golden_live.py from a checkout of the reference)."""
 import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
 
 from audfprint_b200.synth import synth_track, synth_query, pcm_to_float
 from oracle import afp_oracle as orc
+from tests.conftest import GOLDEN
 
-REF = os.environ.get("AFP_REFERENCE", "/root/reference")
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-pytestmark = pytest.mark.skipif(not os.path.isfile(os.path.join(REF, "audfprint_analyze.py")),
-                                reason="live reference not present")
-
-_DRIVER = r'''
-import json, random, sys
-import numpy as np
-sys.path.insert(0, %(root)r); sys.path.insert(0, %(ref)r)
-import audfprint_analyze as an, audfprint_match as ma, audio_read as ar, hash_table as htm
-from audfprint_b200.synth import synth_track, synth_query, pcm_to_float
-pcm = {}
-ar.audio_read = lambda fn, sr=None, channels=None: (pcm_to_float(pcm[fn]), 11025)
-out = {}
-tracks = []
-for seed in %(seeds)r:
-    pcm["t"] = synth_track(seed, 14.0 + seed %% 5)
-    for shifts in (1, 4):
-        a = an.Analyzer(); a.shifts = shifts
-        out["h_%%d_%%d" %% (seed, shifts)] = np.asarray(a.wavfile2hashes("t")).tolist()
-    tracks.append(np.asarray(out["h_%%d_1" %% seed], np.int32))
-random.seed(4)
-ht = htm.HashTable(hashbits=14, depth=6, maxtime=1 << 12)
-for i, h in enumerate(tracks):
-    ht.store("s%%d" %% i, h)
-m = ma.Matcher(); m.window = 2; m.threshcount = 3; m.search_depth = 4
-for j, seed in enumerate(%(seeds)r):
-    q, _ = synth_query(synth_track(seed, 14.0 + seed %% 5), 77 + j, seconds=6.0, noise_sigma=0.01)
-    pcm["q"] = q
-    a = an.Analyzer(); a.shifts = 4
-    qh = np.asarray(a.wavfile2hashes("q"), np.int32)
-    out["q_%%d" %% seed] = qh.tolist()
-    out["hits_%%d" %% seed] = ht.get_hits(qh).tolist()
-    out["rows_%%d" %% seed] = m.match_hashes(ht, qh).tolist()
-out["table"] = ht.table.tolist(); out["counts"] = ht.counts.tolist(); out["hpi"] = np.asarray(ht.hashesperid).tolist()
-print("JSON" + json.dumps(out))
-'''
+FRESH_SEEDS = [5101, 5102, 5103, 5104]
+ANALYZER_PARAMS = [(20.0, 3, 2, 30.0, 5), (20.0, 3, 3, 30.0, 5), (20.0, 3, 8, 30.0, 5), (35.0, 5, 1, 20.0, 3),
+                   (50.0, 6, 4, 30.0, 8), (10.0, 1, 1, 45.0, 1), (70.0, 8, 1, 30.0, 16)]
+MATCHER_PARAMS = [(0, 5, 100, 100), (3, 0, 5, 100), (1, 5, 1, 100), (2, 1, 100, 0), (2, 5, 0, 100), (1, 2, 3, 1)]
+SPREAD_CASES = [(256, 4.0), (256, 30.0), (64, 2.5), (17, 1.0), (300, 12.0), (1, 4.0)]
 
 
-def test_oracle_equals_live_reference_on_fresh_seeds():
-    seeds = [5101, 5102, 5103, 5104]
-    code = _DRIVER % {"root": ROOT, "ref": REF, "seeds": seeds}
-    run = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600)
-    assert run.returncode == 0, run.stderr[-2000:]
-    ref = json.loads([ln for ln in run.stdout.splitlines() if ln.startswith("JSON")][0][4:])
+@pytest.fixture(scope="module")
+def golden_live():
+    return np.load(os.path.join(GOLDEN, "live_reference.npz"))
+
+
+def outputs(g, group):
+    """The stored outputs of one reference run, under the names that run gave them."""
+    return {k[len(group) + 1:]: g[k] for k in g.files if k.startswith(group + "/")}
+
+
+def test_oracle_equals_live_reference_on_fresh_seeds(golden_live):
+    seeds = FRESH_SEEDS
+    ref = outputs(golden_live, "fresh")
     tracks = []
     for seed in seeds:
         d = pcm_to_float(synth_track(seed, 14.0 + seed % 5))
@@ -83,60 +56,12 @@ def test_oracle_equals_live_reference_on_fresh_seeds():
         assert sorted(map(tuple, rows[:, :4])) == sorted(map(tuple, want[:, :4]))        # same alignments
 
 
-_PARAM_DRIVER = r'''
-import json, random, sys
-import numpy as np
-sys.path.insert(0, %(root)r); sys.path.insert(0, %(ref)r)
-import audfprint_analyze as an, audfprint_match as ma, audio_read as ar, hash_table as htm
-from audfprint_b200.synth import synth_track, synth_query, pcm_to_float
-pcm = {}
-ar.audio_read = lambda fn, sr=None, channels=None: (pcm_to_float(pcm[fn]), 11025)
-out = {}
-for k, (density, fanout, shifts, f_sd, maxpks) in enumerate(%(aparams)r):
-    for i in range(2):
-        pcm["t"] = synth_track(6000 + 10 * k + i, 9.0 + i)
-        a = an.Analyzer(density)
-        a.maxpairsperpeak, a.shifts, a.f_sd, a.maxpksperframe = fanout, shifts, f_sd, maxpks
-        out["h_%%d_%%d" %% (k, i)] = np.asarray(a.wavfile2hashes("t")).reshape(-1, 2).tolist()
-        if shifts == 1:
-            out["p_%%d_%%d" %% (k, i)] = np.asarray(a.wavfile2peaks("t")).reshape(-1, 2).tolist()
-# matcher parameters on a small overflowing table
-random.seed(9)
-ht = htm.HashTable(hashbits=12, depth=8, maxtime=1 << 14)
-trk = [synth_track(6500 + i, 12.0) for i in range(12)]
-for i, t in enumerate(trk):
-    pcm["t"] = t
-    ht.store("s%%d" %% i, an.Analyzer().wavfile2hashes("t"))
-out["table"] = ht.table.tolist(); out["counts"] = ht.counts.tolist(); out["hpi"] = np.asarray(ht.hashesperid).tolist()
-qs = []
-for j in range(4):
-    q, _ = synth_query(trk[3 * j], 900 + j, seconds=7.0, noise_sigma=0.01)
-    pcm["q"] = q
-    a = an.Analyzer(); a.shifts = 4
-    qs.append(np.asarray(a.wavfile2hashes("q"), np.int32).reshape(-1, 2))
-    out["q_%%d" %% j] = qs[-1].tolist()
-for k, (window, thresh, sdepth, maxal) in enumerate(%(mparams)r):
-    m = ma.Matcher()
-    m.window, m.threshcount, m.search_depth, m.max_alignments_per_id = window, thresh, sdepth, maxal
-    for j, qh in enumerate(qs):
-        out["rows_%%d_%%d" %% (k, j)] = np.asarray(m.match_hashes(ht, qh)).reshape(-1, 7).tolist()
-print("JSON" + json.dumps(out))
-'''
-
-ANALYZER_PARAMS = [(20.0, 3, 2, 30.0, 5), (20.0, 3, 3, 30.0, 5), (20.0, 3, 8, 30.0, 5), (35.0, 5, 1, 20.0, 3),
-                   (50.0, 6, 4, 30.0, 8), (10.0, 1, 1, 45.0, 1), (70.0, 8, 1, 30.0, 16)]
-MATCHER_PARAMS = [(0, 5, 100, 100), (3, 0, 5, 100), (1, 5, 1, 100), (2, 1, 100, 0), (2, 5, 0, 100), (1, 2, 3, 1)]
-
-
-def test_oracle_equals_live_reference_on_non_default_parameters():
+def test_oracle_equals_live_reference_on_non_default_parameters(golden_live):
     """The parameter settings the GPU tests check against the ORACLE only
     (test_non_default_analyzer_parameters_vs_oracle, test_matcher_edge_parameters_vs_oracle) -
     density / fanout / shifts / f_sd / maxpksperframe and window / threshcount / search_depth /
-    max_alignments_per_id - checked here oracle vs LIVE reference, which closes the chain."""
-    code = _PARAM_DRIVER % {"root": ROOT, "ref": REF, "aparams": ANALYZER_PARAMS, "mparams": MATCHER_PARAMS}
-    run = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=900)
-    assert run.returncode == 0, run.stderr[-2000:]
-    ref = json.loads([ln for ln in run.stdout.splitlines() if ln.startswith("JSON")][0][4:])
+    max_alignments_per_id - checked here oracle vs the reference's outputs, which closes the chain."""
+    ref = outputs(golden_live, "params")
     for k, (density, fanout, shifts, f_sd, maxpks) in enumerate(ANALYZER_PARAMS):
         for i in range(2):
             d = pcm_to_float(synth_track(6000 + 10 * k + i, 9.0 + i))
@@ -161,24 +86,11 @@ def test_oracle_equals_live_reference_on_non_default_parameters():
     assert nexact >= 12
 
 
-def test_spread_local_maxes_equals_reference_spreadpeaksinvector():
+def test_spread_local_maxes_equals_reference_spreadpeaksinvector(golden_live):
     """The stand-alone method north_star names (audfprint_analyze.py:153-160): the oracle function
-    the GPU test compares afp_spread_peaks with, against the live reference's own method."""
-    code = r'''
-import json, sys
-import numpy as np
-sys.path.insert(0, %r)
-import audfprint_analyze as an
-rng = np.random.default_rng(12)
-out = []
-for n, width in [(256, 4.0), (256, 30.0), (64, 2.5), (17, 1.0), (300, 12.0), (1, 4.0)]:
-    v = rng.standard_normal(n) * 3
-    v[rng.integers(0, n, max(1, n // 9))] = 2.0          # plateaus / equal neighbours
-    out.append([n, width, v.tolist(), an.Analyzer().spreadpeaksinvector(v, width).tolist()])
-print("JSON" + json.dumps(out))
-''' % REF
-    run = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
-    assert run.returncode == 0, run.stderr[-2000:]
-    for n, width, v, want in json.loads([ln for ln in run.stdout.splitlines() if ln.startswith("JSON")][0][4:]):
-        got = orc.spread_local_maxes(np.array(v), orc.gaussian_table(n, width))
-        assert np.array_equal(got, np.array(want)), (n, width)
+    the GPU test compares afp_spread_peaks with, against the reference's own method."""
+    for k, (n, width) in enumerate(SPREAD_CASES):
+        v, want = golden_live["spread/%d/v" % k], golden_live["spread/%d/want" % k]
+        assert len(v) == n
+        got = orc.spread_local_maxes(v, orc.gaussian_table(n, width))
+        assert np.array_equal(got, want), (n, width)

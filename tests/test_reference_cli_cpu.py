@@ -4,7 +4,8 @@ audfprint_b200's mirrors - run on precomputed .afpt inputs (host-only path: no G
 compared with the same commands run on the pure reference.  `match` needs the device and is
 covered by the GPU tests through the same classes.
 
-Build container only: the GPU box has no /root/reference (the test skips there).
+The reference's code comes from oracle/_ref/, which build() compiles from a reference checkout, or
+from the checkout named by $AFP_REFERENCE; the tests skip where neither is present.
 docopt is not installed in the image; a small stand-in parses the reference's own USAGE text."""
 import os
 import re
@@ -14,10 +15,12 @@ import sys
 import numpy as np
 import pytest
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.environ.get("AFP_REFERENCE", "/root/reference")
+from oracle import build_ref
 
-pytestmark = pytest.mark.skipif(not os.path.isfile(os.path.join(REF, "audfprint.py")),
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+REF = build_ref.reference_dir()
+
+pytestmark = pytest.mark.skipif(REF is None,
                                 reason="reference checkout not present")
 
 DRIVER = r'''

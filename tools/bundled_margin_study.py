@@ -1,4 +1,4 @@
-"""How far are the decisions made on the bundled real-music fixtures (tests/golden/bundled.npz)
+"""How far are the decisions made on the bundled real-music fixtures (tests/golden/bundled_pcm.npz)
 from flipping?  The CUDA spectrogram differs from NumPy's by last-ulp rounding (|d| ~ 1e-15..1e-13
 of the largest bin; tests assert <= 1e-11).  This CPU study adds complex Gaussian noise of EPS times
 the largest STFT bin to the oracle's STFT and counts fingerprints that change: the committed PCM
@@ -18,7 +18,7 @@ from oracle import afp_oracle as orc      # noqa: E402  (test infrastructure, CP
 
 
 def main():
-    g = np.load(os.path.join(ROOT, "tests", "golden", "bundled.npz"))
+    g = np.load(os.path.join(ROOT, "tests", "golden", "bundled_pcm.npz"))
     sigs = {"query": g["query/pcm"]}
     for k in (0, 4, 8, 12):
         sigs["track%d" % k] = g["track%d/pcm" % k]
