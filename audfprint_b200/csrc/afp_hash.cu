@@ -37,7 +37,7 @@ struct HashArgs {
 // average instead of 61 mostly-empty columns, and no thread is spent on empty slots.
 // The hash slots of `lm` are pre-filled with AFP_NO_HASH by a memset.
 constexpr int LM_THREADS = 256;
-constexpr int PCAP = 11264;   // peak entries per window (col:20 | slot:4 | bin:8)
+constexpr int PCAP = 11264;   // peak entries per window ((col - w0):20 | slot:4 | bin:8)
 
 __global__ void __launch_bounds__(LM_THREADS) afp_landmark_kernel(HashArgs a) {
   __shared__ uint32_t s_pk[PCAP];
@@ -47,6 +47,8 @@ __global__ void __launch_bounds__(LM_THREADS) afp_landmark_kernel(HashArgs a) {
   const int scols = a.item_scols[a.item0 + blockIdx.x];   // last peak column + 1 (:321)
   const int P = a.maxpks, F = a.fanout, tid = threadIdx.x;
   const int64_t base = it.frame_base;
+  // Columns are stored relative to the window start: a window spans at most W + targetdt < 2^20 columns,
+  // while an item may have any int32 number of frames.
   const int W = max(64, PCAP / P - a.targetdt - 1);       // source columns per window
   for (int w0 = 0; w0 < scols; w0 += W) {
     const int wend = min(scols, w0 + W + a.targetdt);     // sources in [w0, w0+W), targets up to +targetdt
@@ -65,7 +67,7 @@ __global__ void __launch_bounds__(LM_THREADS) afp_landmark_kernel(HashArgs a) {
       }
       const int at = s_run + s_scan[tid] - n;
       for (int k = 0; k < n; ++k)
-        s_pk[at + k] = ((uint32_t)c << 12) | ((uint32_t)k << 8) | a.pk_bin[(base + c) * P + k];
+        s_pk[at + k] = ((uint32_t)(c - w0) << 12) | ((uint32_t)k << 8) | a.pk_bin[(base + c) * P + k];
       __syncthreads();
       if (tid == LM_THREADS - 1) s_run += s_scan[tid];
       __syncthreads();
@@ -73,14 +75,14 @@ __global__ void __launch_bounds__(LM_THREADS) afp_landmark_kernel(HashArgs a) {
     const int np = s_run;
     for (int i = tid; i < np; i += LM_THREADS) {
       const uint32_t e = s_pk[i];
-      const int col = (int)(e >> 12), slot = (int)((e >> 8) & 15), b1 = (int)(e & 255);
+      const int col = w0 + (int)(e >> 12), slot = (int)((e >> 8) & 15), b1 = (int)(e & 255);
       if (col >= w0 + W) break;                           // entries are column-sorted: only targets remain
       uint32_t* out = a.lm + ((base + col) * P + slot) * F;
       const int c2lo = col + a.mindt, c2hi = min(scols, col + a.targetdt);     // :331-332
       int n = 0;
       for (int j = (a.mindt > 0) ? i + 1 : i - slot; j < np && n < F; ++j) {
         const uint32_t t = s_pk[j];
-        const int c2 = (int)(t >> 12);
+        const int c2 = w0 + (int)(t >> 12);
         if (c2 >= c2hi) break;
         if (c2 < c2lo) continue;
         const int b2 = (int)(t & 255);

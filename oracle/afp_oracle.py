@@ -234,9 +234,11 @@ def shift_offsets(shifts: int, n_hop: int = N_HOP):
 
 
 def fingerprint(d: np.ndarray, density: float = 20.0, fanout: int = 3, shifts: int = 1,
-                f_sd: float = 30.0, maxpks: int = 5) -> np.ndarray:
+                f_sd: float = 30.0, maxpks: int = 5, mindt: int = 2, targetdt: int = 63,
+                targetdf: int = 31) -> np.ndarray:
     """PCM (float) -> int32 (U,2) rows [time, hash], sorted by (time, hash),
     duplicates across shifts removed.  audfprint_analyze.py:369-377, 401-422.
+    mindt / targetdt / targetdf are the Analyzer attributes of the pairing window (:139-143).
     Returns an empty (0,2) array where the reference returns [] (:401-402)."""
     lists = []
     if shifts < 2:
@@ -246,7 +248,8 @@ def fingerprint(d: np.ndarray, density: float = 20.0, fanout: int = 3, shifts: i
             lists.append(find_peaks(d[off:], density, f_sd, maxpks))
     if shifts < 2 and len(lists[0]) == 0:
         return np.zeros((0, 2), np.int32)
-    rows = np.concatenate([landmarks_to_hashes(peaks_to_landmarks(pl, fanout)) for pl in lists])
+    rows = np.concatenate([landmarks_to_hashes(peaks_to_landmarks(pl, fanout, mindt, targetdt, targetdf))
+                           for pl in lists])
     key = (rows[:, 0].astype(np.uint64) << np.uint64(32)) + rows[:, 1].astype(np.uint64)
     key = np.unique(key)
     return np.stack([key >> np.uint64(32), key & np.uint64(0xFFFFFFFF)], axis=1).astype(np.int32)

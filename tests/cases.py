@@ -81,3 +81,60 @@ LONG_HASHBITS = 16
 LONG_DEPTH = 20
 LONG_MAXTIMEBITS = 12
 LONG_QUERIES = [(0, 10.0), (1, 10.0), (2, 10.0), (1, 170.0)]      # (track index, seconds)
+
+# K3 pairing window at its limits (oracle/make_golden_pairing.py, tests/test_gpu_landmarks.py).
+# (mindt, targetdt, targetdf, fanout, maxpks, shifts, density, f_sd); densities are high enough that
+# columns fill up to maxpks peaks
+PAIRING_SETTINGS = [
+    (0, 63, 31, 3, 5, 1, 20.0, 30.0),       # same-column pairs and self-pairs
+    (0, 64, 32, 16, 16, 1, 1000.0, 3.0),    # both 6-bit fields at their limit; merge buffer full
+    (0, 64, 32, 4, 16, 4, 2000.0, 2.0),     # merge buffer full across shifts
+    (2, 63, 31, 1, 16, 16, 1000.0, 3.0),    # 16 shifts
+    (63, 64, 32, 2, 8, 2, 60.0, 30.0),      # only dt = 63
+    (1, 3, 4, 2, 5, 4, 40.0, 30.0),         # narrowest useful window
+    (5, 20, 10, 4, 8, 3, 40.0, 30.0),       # 3 shifts: int16 shift items start off 16-byte boundaries
+]
+PAIRING_SEED = 7113
+PAIRING_SECONDS = 8.0
+
+
+def gapped_track(seed: int, seconds: float) -> np.ndarray:
+    """synth_track with digital silence of 40..63 frames between bursts of 4..29 frames: isolated
+    peak clusters whose pairs span the whole pairing window."""
+    x = synth_track(seed, seconds).copy()
+    rng = np.random.default_rng(seed + 1)
+    c = int(rng.integers(20, 40))
+    while c * 256 < len(x):
+        g = int(rng.integers(40, 64))
+        x[c * 256:(c + g) * 256] = 0
+        c += g + int(rng.integers(4, 30))
+    return x
+
+
+def pairing_tracks():
+    """The two int16 tracks every pairing setting is run on."""
+    return [synth_track(PAIRING_SEED, PAIRING_SECONDS), gapped_track(PAIRING_SEED, PAIRING_SECONDS)]
+
+
+# explicit peak lists for peaks2landmarks: (mindt, targetdt, targetdf, fanout, maxpks), and first columns
+# on both sides of 2^20, 2^21 and 2^22
+PEAK_LIST_SETTINGS = [(2, 63, 31, 3, 5), (0, 64, 32, 8, 16)]
+PEAK_LIST_STARTS = [0, (1 << 20) - 300, (1 << 20) + 1000, (1 << 21) + 5, (1 << 22) - 100]
+PEAK_LIST_COLUMNS = 400
+
+
+def peak_list(seed: int, start: int, maxpks: int, ncols: int = PEAK_LIST_COLUMNS) -> np.ndarray:
+    """int32 (n, 2) rows (col, bin), column-major, bins ascending, in columns [start, start + ncols):
+    full columns of maxpks peaks, empty stretches longer than any pairing window, and a lone final
+    peak after a gap."""
+    rng = np.random.default_rng(seed)
+    counts = rng.integers(0, maxpks + 1, ncols)
+    counts[rng.random(ncols) < 0.15] = maxpks
+    for g0 in (ncols // 4, ncols // 2 + 13):
+        counts[g0:g0 + 70 + int(rng.integers(0, 10))] = 0
+    counts[ncols - 40:] = 0
+    counts[0] = maxpks
+    counts[-1] = 1
+    rows = [(start + c, int(b)) for c in range(ncols)
+            for b in np.sort(rng.choice(256, int(counts[c]), replace=False))]
+    return np.array(rows, np.int32).reshape(-1, 2)
